@@ -269,6 +269,32 @@ def _eager_gpu_legs(mref, why, sd, frames_dev, model, dev, F_):
     return eager, parity
 
 
+DUMP_BUDGET = 64_000_000           # bytes written by --dump-outputs at most
+
+
+def _host_outputs(out):
+    """name -> float32 host array of what `Spann3R.forward` returned: preds[i][k] and the res2 half of preds_all[i]
+    (their res1 halves are the preds entries themselves)."""
+    preds, preds_all = out
+    arrays = {f"preds_{i}_{k}": v for i, p in enumerate(preds) for k, v in p.items()}
+    arrays.update({f"preds_all_{i}_res2_{k}": v for i, (_, r2) in enumerate(preds_all) for k, v in r2.items()})
+    return {n: v.detach().float().cpu().numpy() for n, v in arrays.items()}
+
+
+def _write_outputs(arrays, out_dir):
+    """DIR/<name>.npy; above DUMP_BUDGET every array keeps the same fraction of its elements, at indices drawn with a
+    fixed seed (flattened, ascending), so the files of two runs line up element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    budget = DUMP_BUDGET - 256 * len(arrays)         # room for the .npy headers
+    for name, a in arrays.items():
+        if total > budget:
+            m = max(1, a.size * budget // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, m, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -293,7 +319,14 @@ def main():
                     "random-init checkpoint, SURVEY.md §8d: report both)")
     ap.add_argument("--batch", type=int, default=1,
                     help="sequences advanced in lockstep per GPU (BASELINE config[2] runs 8 per GPU); the headline is 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy in float32: "
+                         "preds_<frame>_<key> and preds_all_<frame>_res2_<key>.  The inputs are seeded, so two builds run with "
+                         "the same arguments can be compared file by file.  Above 64 MB in all, every array is reduced to the "
+                         "same fixed, seeded sample of its elements")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -310,7 +343,7 @@ def main():
     from spann3r_b200 import Spann3R, synth
 
     W_ = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     F_ = args.frames
     sd = synth.make_state_dict(sharpen=not args.raw_checkpoint)
     model = Spann3R(dus3r_name=None)
@@ -356,10 +389,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(K):
-        model(resident[i % n_distinct])
+        out_last = model(resident[i % n_distinct])
     e1.record()
     barrier()
     ms = max_over_ranks(e0.elapsed_time(e1))
+    # copied out before anything else runs on the model: its outputs may live in buffers the next call reuses
+    dumped = _host_outputs(out_last) if args.dump_outputs and rank == 0 else None
+    del out_last
     launches = eng.take_launches()
     flops_issued = eng.take_flops()
     # the sampler stops HERE: nvidia-smi polling the driver every 100 ms costs the e2e loop below a third of its throughput
@@ -508,6 +544,8 @@ def main():
         model.norm_q.weight.data.mul_(8.0)
         model.invalidate_packed()
 
+    if dumped is not None:
+        _write_outputs(dumped, args.dump_outputs)
     if rank == 0:
         print(json.dumps({
             "reference_eager_gpu": eager, "parity_vs_reference_in_run": parity_ref, "raw_checkpoint": raw, "config3": config3,

@@ -56,8 +56,9 @@ def test_forward_matches_reference_golden(models, fname, sharpen, nf, H, W):
         for k, v in r2.items():
             errs[f"preds_all/{i}/res2/{k}"] = rel_l2(v[:, ::s, ::s].cpu(), g[f"preds_all/{i}/res2/{k}"])
     assert all(bool(torch.isfinite(v).all()) for p in preds for v in p.values())
-    errs["mem_k"] = rel_l2(mem.mem_k[:, ::7, ::8].cpu(), g["mem/mem_k_sub"])
-    errs["mem_v"] = rel_l2(mem.mem_v[:, ::7, ::8].cpu(), g["mem/mem_v_sub"])
+    t = int(g["meta/tok_stride"])
+    errs["mem_k"] = rel_l2(mem.mem_k[:, ::t, ::8].cpu(), g["mem/mem_k_sub"])
+    errs["mem_v"] = rel_l2(mem.mem_v[:, ::t, ::8].cpu(), g["mem/mem_v_sub"])
     errs["mem_attn"] = rel_l2(mem.mem_attn.cpu(), g["mem/mem_attn"])
     print({k: f"{v:.2e}" for k, v in errs.items()})
     assert np.array_equal(mem.mem_count.cpu().numpy(), g["mem/mem_count"])
@@ -85,7 +86,7 @@ def test_mem_pos_enc_variant_matches_reference_golden():
     preds, _, mem = m(synth.make_frames(3, 224, 224), return_memory=True)
     s = int(g["meta/px_stride"])
     errs = {f"{i}/{k}": rel_l2(v[:, ::s, ::s].cpu(), g[f"preds/{i}/{k}"]) for i, p in enumerate(preds) for k, v in p.items()}
-    errs["mem_v"] = rel_l2(mem.mem_v[:, ::7, ::8].cpu(), g["mem/mem_v_sub"])
+    errs["mem_v"] = rel_l2(mem.mem_v[:, ::int(g["meta/tok_stride"]), ::8].cpu(), g["mem/mem_v_sub"])
     print({k: f"{v:.2e}" for k, v in errs.items()})
     assert max(errs.values()) < TOL, errs
     del m
@@ -309,11 +310,12 @@ def test_offline_reconstruction_matches_reference_golden(models):
     with contextlib.redirect_stdout(io.StringIO()):
         preds, preds_all, idx_used = m.offline_reconstruction(frames, graph)
     assert list(idx_used) == list(g["idx_used"])
+    s = int(g["meta/px_stride"])
     errs = {}
     for i, p in enumerate(preds):
         assert set(p.keys()) == {k.split("/")[-1] for k in g.files if k.startswith(f"preds/{i}/")}
         for k, v in p.items():
-            errs[f"{i}/{k}"] = rel_l2(v.cpu(), g[f"preds/{i}/{k}"])
+            errs[f"{i}/{k}"] = rel_l2(v[:, ::s, ::s].cpu(), g[f"preds/{i}/{k}"])
     print({k: "%.1e" % v for k, v in errs.items()})
     assert max(errs.values()) < TOL, errs
 

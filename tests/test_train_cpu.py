@@ -172,8 +172,10 @@ class _TorchEngine:
 
 def test_training_forward_and_recompute_backward_end_to_end_on_cpu(monkeypatch, sd):
     """`train.forward_train` (the real frame loop, stage Functions and parameter routing) over a torch stand-in engine:
-    outputs equal the oracle's training-branch forward and the gradients equal autograd through the oracle to fp32 rounding.
-    (On the GPU the same backward is fed by the CUDA forward, whose activations differ by <= 3e-4: tests/test_train_gpu.py.)"""
+    outputs equal the oracle's training-branch forward and the gradients equal autograd through the oracle.
+    (On the GPU the same backward is fed by the CUDA forward, whose activations differ by <= 3e-4: tests/test_train_gpu.py.)
+    Both sides run in float64: in fp32 their gradients differ by 2e-4 .. 4e-4 depending on the host's CPU kernels and
+    thread count, rounding noise of the same size as the bound; in float64 they agree to ~1e-15."""
     from spann3r_b200 import Spann3R
     import spann3r_b200.engine as E
 
@@ -181,16 +183,17 @@ def test_training_forward_and_recompute_backward_end_to_end_on_cpu(monkeypatch, 
         def __init__(self, batch, cap, device):
             self.len, self.cap = 0, cap
     monkeypatch.setattr(E, "MemoryBank", _Bank)
-    m = Spann3R(dus3r_name=None, memory_dropout=0.0)
+    sd = {k: v.double() for k, v in sd.items()}
+    m = Spann3R(dus3r_name=None, memory_dropout=0.0).double()
     m.load_state_dict(sd, strict=True)
     m.train()
     P = dict(m.named_parameters(remove_duplicate=False))
     eng = _TorchEngine({k: v.detach() for k, v in P.items()}, 1, H, W)
     monkeypatch.setattr(m, "_engine_for", lambda *a, **k: eng)
     monkeypatch.setattr(m, "_dev", lambda t: t)
-    frames = synth.make_frames(3, H, W)
+    frames = [{"img": f["img"].double()} for f in synth.make_frames(3, H, W)]
     g = torch.Generator().manual_seed(5)
-    wts = [torch.randn(1, H, W, 3, generator=g) for _ in range(3)]
+    wts = [torch.randn(1, H, W, 3, generator=g, dtype=torch.float64) for _ in range(3)]
 
     def loss_of(preds):
         tot = 0.0
@@ -213,4 +216,5 @@ def test_training_forward_and_recompute_backward_end_to_end_on_cpu(monkeypatch, 
             assert rel_l2(p[k].detach(), r[k].detach()) < 1e-5, k
     grads = torch.autograd.grad(loss_of(ref), [sdr[k] for k in watch])
     errs = {k: rel_l2(got[k], gr) for k, gr in zip(watch, grads)}
+    assert all(got[k].dtype == torch.float64 for k in watch)
     assert max(errs.values()) < 2e-4, errs

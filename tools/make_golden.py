@@ -10,17 +10,21 @@ fixtures it writes into tests/golden/.
 
 Outputs
   spann3r_b200/state_dict_spec.json   key -> shape of the reference Spann3R state dict
-  tests/golden/cfg1_224_2f_raw.npz    BASELINE config 1 (2 x 224x224), raw random-init weights
-  tests/golden/seq_224_4f_sharp.npz   4 x 224x224, sharpened weights (two memory reads)
-  tests/golden/seq_384x512_3f_sharp.npz  3 x 384x512, sharpened, outputs sub-sampled (::4, ::4)
-  tests/golden/offline_224_4f_sharp.npz  offline mode: 4 x 224x224, complete pair graph -> offline_reconstruction
-  tests/golden/seq_288x224_4f_sharp.npz  PORTRAIT 4 x (H=288, W=224): transpose_to_landscape (dust3r/utils/misc.py:66-94), outputs (::2, ::2)
-  tests/golden/seq_512x384_3f_sharp.npz  PORTRAIT 3 x (H=512, W=384), outputs sub-sampled (::4, ::4)
-  tests/golden/seq_224_3f_sharp_mempos.npz  3 x 224x224 with Spann3R(mem_pos_enc=True) (RoPE inside the value encoder)
-  tests/golden/cfg2_384x512_10f_sharp.npz  BASELINE config 2 exactly (10 x 384x512, sharpened ckpt), outputs (::8, ::8)   [--only cfg2]
-  tests/golden/cfg2_384x512_10f_raw.npz    the same on the RAW random-init checkpoint (SURVEY 8d: report both)            [--only cfg2]
-Each npz also holds sub-sampled per-stage activations captured with forward hooks so that a
-parity failure can be localised to a stage.
+  tests/golden/cfg1_224_2f_raw.npz    BASELINE config 1 (2 x 224x224), raw random-init weights, outputs (::3, ::3)
+  tests/golden/seq_224_4f_sharp.npz   4 x 224x224, sharpened weights (two memory reads), outputs (::3, ::3)
+  tests/golden/seq_384x512_3f_sharp.npz  3 x 384x512, sharpened, outputs sub-sampled (::12, ::12), tokens ::21
+  tests/golden/offline_224_4f_sharp.npz  offline mode: 4 x 224x224, complete pair graph -> offline_reconstruction, outputs (::3, ::3)
+  tests/golden/seq_288x224_4f_sharp.npz  PORTRAIT 4 x (H=288, W=224): transpose_to_landscape (dust3r/utils/misc.py:66-94), outputs (::6, ::6)
+  tests/golden/seq_512x384_3f_sharp.npz  PORTRAIT 3 x (H=512, W=384), outputs sub-sampled (::12, ::12)
+  tests/golden/seq_224_3f_sharp_mempos.npz  3 x 224x224 with Spann3R(mem_pos_enc=True) (RoPE inside the value encoder), outputs (::6, ::6)
+  tests/golden/cfg2_384x512_10f_sharp.npz  BASELINE config 2 exactly (10 x 384x512, sharpened ckpt), outputs (::16, ::16), tokens ::21   [--only cfg2]
+  tests/golden/cfg2_384x512_10f_raw.npz    the same on the RAW random-init checkpoint (SURVEY 8d: report both)                           [--only cfg2]
+Each npz also holds sub-sampled per-stage activations (first call of each hooked module) captured with forward hooks
+so that a parity failure can be localised to a stage.
+
+Every file stays under 1 MB.  Output maps are sub-sampled with a pixel stride (`meta/px_stride`) of at most the
+16-pixel patch, so every patch contributes samples; memory keys / values and token activations keep every
+`meta/tok_stride`-th token and every 8th channel.
 """
 import argparse
 import json
@@ -73,11 +77,11 @@ def sub(t, tok_stride=7, ch_stride=8):
     if t.ndim == 3:      # [B, N, C] tokens
         return t[:, ::tok_stride, ::ch_stride].contiguous().numpy()
     if t.ndim == 4:      # [B, C, H, W] feature map
-        return t[:, ::ch_stride, ::3, ::3].contiguous().numpy()
+        return t[:, ::ch_stride, ::9, ::9].contiguous().numpy()
     return t.numpy()
 
 
-def run(model, frames, out_path, px_stride=1, hooks=True):
+def run(model, frames, out_path, px_stride=1, tok_stride=7, hooks=True):
     acts = {}
     handles = []
     if hooks:
@@ -106,9 +110,9 @@ def run(model, frames, out_path, px_stride=1, hooks=True):
         for name, pick in watch.items():
             def mk(name, pick):
                 def hook(_m, _i, o):
-                    k = "act/" + name
-                    n = sum(1 for kk in acts if kk.startswith(k + "#"))
-                    acts[f"{k}#{n}"] = sub(pick(o))
+                    k = "act/" + name + "#0"
+                    if k not in acts:
+                        acts[k] = sub(pick(o), tok_stride=tok_stride)
                 return hook
             handles.append(mods[name].register_forward_hook(mk(name, pick)))
     t0 = time.time()
@@ -125,11 +129,12 @@ def run(model, frames, out_path, px_stride=1, hooks=True):
     for i, (r1, r2) in enumerate(preds_all):
         for k, v in r2.items():
             out[f"preds_all/{i}/res2/{k}"] = v[:, ::s, ::s].contiguous().numpy()
-    out["mem/mem_k_sub"] = sub(mem.mem_k)
-    out["mem/mem_v_sub"] = sub(mem.mem_v)
+    out["mem/mem_k_sub"] = sub(mem.mem_k, tok_stride=tok_stride)
+    out["mem/mem_v_sub"] = sub(mem.mem_v, tok_stride=tok_stride)
     out["mem/mem_attn"] = mem.mem_attn.numpy()
     out["mem/mem_count"] = mem.mem_count.numpy()
     out["meta/px_stride"] = np.array(s)
+    out["meta/tok_stride"] = np.array(tok_stride)
     out["meta/ref_seconds"] = np.array(dt)
     out["meta/threads"] = np.array(torch.get_num_threads())
     finite = all(np.isfinite(v).all() for k, v in out.items() if k.startswith("preds"))
@@ -140,7 +145,7 @@ def run(model, frames, out_path, px_stride=1, hooks=True):
           f"{os.path.getsize(out_path)/1e6:.2f} MB")
 
 
-def run_offline(model, frames, out_path):
+def run_offline(model, frames, out_path, px_stride=3):
     """demo.py:104-118 offline branch: make_pairs (complete, symmetrized) -> dust3r.inference.inference -> offline_reconstruction."""
     from dust3r.image_pairs import make_pairs  # noqa (reference)
     from dust3r.inference import inference  # noqa (reference)
@@ -155,11 +160,11 @@ def run_offline(model, frames, out_path):
            "graph/view2_idx": np.array(output["view2"]["idx"]),
            "graph/pred1_conf": output["pred1"]["conf"][:, ::4, ::4].contiguous().numpy(),
            "graph/pred2_conf": output["pred2"]["conf"][:, ::4, ::4].contiguous().numpy(),
-           "graph/pred1_pts3d": output["pred1"]["pts3d"][:, ::4, ::4].contiguous().numpy(),
-           "meta/ref_seconds": np.array(time.time() - t0)}
+           "meta/ref_seconds": np.array(time.time() - t0), "meta/px_stride": np.array(px_stride)}
+    s = px_stride
     for i, p in enumerate(preds):
         for k, v in p.items():
-            out[f"preds/{i}/{k}"] = v.contiguous().numpy()
+            out[f"preds/{i}/{k}"] = v[:, ::s, ::s].contiguous().numpy()
     np.savez_compressed(out_path, **out)
     print(f"wrote {out_path}: idx_used={idx_used}, {time.time() - t0:.1f}s, {os.path.getsize(out_path)/1e6:.2f} MB")
 
@@ -174,28 +179,30 @@ def main():
     if args.only in ("all", "spec", "cfg1"):
         m = build_reference(sharpen=False)
         if args.only != "spec":
-            run(m, synth.make_frames(2, 224, 224), os.path.join(GOLD, "cfg1_224_2f_raw.npz"))
+            run(m, synth.make_frames(2, 224, 224), os.path.join(GOLD, "cfg1_224_2f_raw.npz"), px_stride=3)
         del m
     if args.only in ("all", "mempos"):
         m = build_reference(sharpen=True, mem_pos_enc=True)
-        run(m, synth.make_frames(3, 224, 224), os.path.join(GOLD, "seq_224_3f_sharp_mempos.npz"), px_stride=2, hooks=False)
+        run(m, synth.make_frames(3, 224, 224), os.path.join(GOLD, "seq_224_3f_sharp_mempos.npz"), px_stride=6, hooks=False)
         del m
     if args.only in ("all", "cfg2"):   # the headline config itself, both checkpoints (~10 CPU-minutes each on 8 cores)
         for sharpen, tag in ((True, "sharp"), (False, "raw")):
             m = build_reference(sharpen=sharpen)
-            run(m, synth.make_frames(10, 384, 512), os.path.join(GOLD, f"cfg2_384x512_10f_{tag}.npz"), px_stride=8, hooks=False)
+            # px 16 = one sample per patch: with stride 8, ten frames plus the memory would not fit in 1 MB
+            run(m, synth.make_frames(10, 384, 512), os.path.join(GOLD, f"cfg2_384x512_10f_{tag}.npz"), px_stride=16,
+                tok_stride=21, hooks=False)
             del m
     if args.only in ("all", "seq224", "seq512", "offline", "portrait"):
         m = build_reference(sharpen=True)
         if args.only in ("all", "portrait"):
-            run(m, synth.make_frames(4, 288, 224), os.path.join(GOLD, "seq_288x224_4f_sharp.npz"), px_stride=2, hooks=False)
-            run(m, synth.make_frames(3, 512, 384), os.path.join(GOLD, "seq_512x384_3f_sharp.npz"), px_stride=4, hooks=False)
+            run(m, synth.make_frames(4, 288, 224), os.path.join(GOLD, "seq_288x224_4f_sharp.npz"), px_stride=6, hooks=False)
+            run(m, synth.make_frames(3, 512, 384), os.path.join(GOLD, "seq_512x384_3f_sharp.npz"), px_stride=12, hooks=False)
         if args.only in ("all", "offline"):
             run_offline(m, synth.make_frames(4, 224, 224), os.path.join(GOLD, "offline_224_4f_sharp.npz"))
         if args.only in ("all", "seq224"):
-            run(m, synth.make_frames(4, 224, 224), os.path.join(GOLD, "seq_224_4f_sharp.npz"))
+            run(m, synth.make_frames(4, 224, 224), os.path.join(GOLD, "seq_224_4f_sharp.npz"), px_stride=3)
         if args.only in ("all", "seq512"):
-            run(m, synth.make_frames(3, 384, 512), os.path.join(GOLD, "seq_384x512_3f_sharp.npz"), px_stride=4)
+            run(m, synth.make_frames(3, 384, 512), os.path.join(GOLD, "seq_384x512_3f_sharp.npz"), px_stride=12, tok_stride=21)
 
 
 if __name__ == "__main__":
